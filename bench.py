@@ -59,7 +59,13 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the short GRM / PCA / LD measurements reported under `secondary`")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of the KING pairs (counts and kinship) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # ----------------------------------------------------------------------------------- synthetic data
@@ -404,8 +410,8 @@ def secondary_legs(args, torch, p, ctx, dev, peak_tops):
                      "seconds": dt, "pairs_per_s": pairs / dt, "achieved": 12 * pairs * nf / dt / 1e12, "unit": "TOP/s (int8; 6 products x 2 ops per pair and founder)", "peak": peak_tops,
                      "frac": (12 * pairs * nf / dt / 1e12) / peak_tops if peak_tops else None}
         del g4, flags_t
-        ref = ref_binary()
-        if ref:
+        ref = os.path.join(ROOT, "oracle", "_ref", "plink2")
+        if os.path.exists(ref):
             nc, mc = 8192, 32768
             tmp = tempfile.mkdtemp(prefix="pl2ld_")
             try:
@@ -442,8 +448,8 @@ def secondary_legs(args, torch, p, ctx, dev, peak_tops):
         sec["score"] = {"kernel": "score_kernel", "workload": f"--score accumulation, {ns} samples x {ms} scored entries, genotypes resident (whole pl2gpu_score_add_variants call)", "seconds": dt,
                         "sample_entries_per_s": ns * ms / dt, "achieved": ns * ms / 4 / dt / 1e9, "unit": "GB/s of 2-bit genotypes", "peak": hbm_peak_gbs(), "bound": "ALU (fp64 table add per sample and entry), then HBM"}
         del g5
-        ref = ref_binary()
-        if ref:
+        ref = os.path.join(ROOT, "oracle", "_ref", "plink2")
+        if os.path.exists(ref):
             nc, mc = 8192, 65536
             tmp = tempfile.mkdtemp(prefix="pl2sc_")
             try:
@@ -461,6 +467,32 @@ def secondary_legs(args, torch, p, ctx, dev, peak_tops):
     except Exception as ex:
         sec.setdefault("score", {})["error"] = str(ex)[-300:]
     return sec
+
+
+# ------------------------------------------------------------------------------------- outputs
+DUMP_ROWS, DUMP_COLS = 64, 4096
+
+
+def dump_outputs(job, r0, r1, out_dir):
+    """What a caller of the timed KingJob receives after the last timed step: uint32 counts[pair][5] and fp64 kinship.
+    The whole triangle does not fit a comparable dump, so a fixed sample: DUMP_ROWS rows of [r0, r1) and up to
+    DUMP_COLS columns of each, drawn by a seeded generator.  Every array is float64 (counts and indices are exact)."""
+    import numpy as np
+
+    rng = np.random.default_rng(0)
+    lo = max(r0, 1)  # row 0 has no pairs
+    rows = np.sort(rng.choice(np.arange(lo, r1), size=min(DUMP_ROWS, r1 - lo), replace=False))
+    row_idx, col_idx, counts, kinship = [], [], [], []
+    for r in rows:
+        r = int(r)
+        cols = np.sort(rng.choice(r, size=min(DUMP_COLS, r), replace=False))
+        row_idx.append(np.full(cols.size, r))
+        col_idx.append(cols)
+        counts.append(job.counts(r, r + 1)[cols])  # row r holds the pairs (r, 0..r-1)
+        kinship.append(job.kinship(r, r + 1)[cols])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, parts in (("king_pair_row", row_idx), ("king_pair_col", col_idx), ("king_counts", counts), ("king_kinship", kinship)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.concatenate(parts).astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------- B200 arm
@@ -551,6 +583,9 @@ def b200_arm(args):
     step_ms = float(t_ms[0].item()) / args.steps
     kern_ms_max = float(t_ms[1].item())
     value = total_pairs * (mb / 1e6) / (step_ms * 1e-3)
+    # before the e2e leg, which adds more variants to the same job; multi-GPU runs dump rank 0's row block
+    if args.dump_outputs and rank == 0:
+        dump_outputs(job, r0, r1, args.dump_outputs)
 
     # ---- e2e: host buffers through the C-ABI, H2D + D2H inside the timed region ----
     e2e = None

@@ -129,9 +129,11 @@ awk 'BEGIN{OFS="\t"} {if ($1=="XY") $1="chrUn_KI270"; if ($1=="MT" && ++k<=50) $
 $P --bed x.bed --bim x_contigs.bim --fam x.fam --allow-extra-chr --not-chr 1,X --make-bed --threads 2 --out $T/e1 > /dev/null; cp $T/e1.bim x_contigs_sub.bim
 $P --bed x.bed --bim x_contigs.bim --fam x.fam --allow-extra-chr --not-chr X,Y,MT --indep-pairwise 50 5 0.2 --threads 2 --out $T/e2 > /dev/null; cp $T/e2.prune.in x_contigs.prune.in
 $P --bed x.bed --bim x_contigs.bim --fam x.fam --allow-extra-chr --make-king-table --threads 2 --out $T/e3 > /dev/null; gzip -9 -n -c $T/e3.kin0 > x_contigs.kin0.gz
-# --make-pgen: the reference's .pvar / .psam text (its .pgen is compressed differently and not compared) + the .bed of the same view
+# --make-pgen: the reference's .pvar / .psam text, its fixed-width .pgen (format=2; the default mode is compressed
+# differently and not compared) + the .bed of the same view
 $P --bfile x --keep x_keep1.txt x_keep2.txt --extract x_extract.txt --make-pgen --threads 2 --out $T/mp > /dev/null; cp $T/mp.pvar x_mp.pvar; cp $T/mp.psam x_mp.psam
 $P --bfile x --keep x_keep1.txt x_keep2.txt --extract x_extract.txt --make-bed --threads 2 --out $T/mb > /dev/null; cp $T/mb.bed x_mp.bed
+$P --bfile x --keep x_keep1.txt x_keep2.txt --extract x_extract.txt --make-pgen format=2 --threads 2 --out $T/mpf2 > /dev/null; cp $T/mpf2.pgen x_mp.pgen
 $P --pedmap p --make-pgen --threads 2 --out $T/pp > /dev/null; cp $T/pp.pvar p_mp.pvar; cp $T/pp.psam p_mp.psam
 $P --bfile x --bp-space 7 --maf 0.05 --chr 1,X,MT --make-bed --threads 2 --out $T/bs > /dev/null; cp $T/bs.bim x_bpspace.bim   # --bp-space runs after the frequency thresholds
 # --missing: written after the sample filters (incl. --mind) and before the variant thresholds

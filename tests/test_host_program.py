@@ -1,6 +1,8 @@
 """CPU: host-side pieces of plink2_b200 that need no GPU - the pgenlib reader surface (all three
 storage modes incl. difflist / LD-compressed records) and byte-identical number formatting."""
 import gzip
+import hashlib
+import json
 import os
 import subprocess
 
@@ -72,29 +74,12 @@ def test_dtoa_g_matches_reference_text(golden_dir, tmp_path):
     assert got[len(kin)] == "0" and got[len(kin) + 3] == "0.5" and got[len(kin) + 7] == "1e-05"
 
 
-REF_INC = "/root/reference/2.0/include"
-SFMT_OBJ = os.path.join(ROOT, "oracle", "_ref", "obj", "include_SFMT_c.o")
-STRING_OBJS = [os.path.join(ROOT, "oracle", "_ref", "obj", "include_plink2_%s_cc.o" % x) for x in ("string", "base", "bits", "float", "simd")]
+SFMT_DRAWS = 5000
 
 
-@pytest.mark.skipif(not (os.path.isdir(REF_INC) and all(os.path.exists(o) for o in STRING_OBJS)), reason="needs the reference's compiled plink2_string.cc (this container only)")
-def test_dtoa_g_p8_matches_reference_function(tmp_path):
-    """The 8-digit formatter behind --make-grm-sparse, byte for byte against the reference's own dtoa_g_p8
-    (2.0/include/plink2_string.cc:2641) on 85,000 doubles: all magnitude ranges, exact .5 ties at every digit
-    position and values a few 1e-7 either side of them, zeros, infinities, NaN."""
-    harness = tmp_path / "h.cc"
-    harness.write_text(r"""
-#include <cstdio>
-#include "plink2_string.h"
-int main(int argc, char** argv) {
-  FILE* in = fopen(argv[1], "rb"); FILE* out = fopen(argv[2], "w");
-  double x; char buf[64];
-  while (fread(&x, 8, 1, in) == 1) { char* e = plink2::dtoa_g_p8(x, buf); *e = 0; fprintf(out, "%s\n", buf); }
-  fclose(in); fclose(out); return 0;
-}
-""")
-    exe = tmp_path / "h"
-    subprocess.run(["g++", "-O1", "-std=c++11", "-mavx2", "-mbmi", "-mbmi2", "-mfma", "-mlzcnt", "-w", "-I" + REF_INC, "-I/root/reference/2.0/simde", str(harness)] + STRING_OBJS + ["-o", str(exe)], check=True)
+def dtoa_p8_inputs():
+    """85,030 doubles: all magnitude ranges, exact .5 ties at every digit position and values a few 1e-7 either side
+    of them, zeros, infinities, NaN."""
     rng = np.random.default_rng(5)
     fixed = [0.0, -0.0, 1.0, -1.0, 0.5, 0.1, 0.01, 0.001, 0.0001, 1e-5, 123456.789, 12345678.9, 99999999.4, 99999999.5, 1e8, 1.5e8, 9.9999999e-5, 2 / 3, 1 / 3, np.pi, 1e300,
              -2.5e-300, np.inf, -np.inf, np.nan, 0.99999999, 0.999999995, 0.05, 0.025, 0.0125]
@@ -102,50 +87,33 @@ int main(int argc, char** argv) {
         rng.uniform(-1, 1, 20000), 10 ** rng.uniform(-12, 12, 20000) * rng.choice([-1, 1], 20000), rng.uniform(0, 0.2, 20000),
         (rng.integers(1, 10 ** 8, 20000) + 0.5) / 10.0 ** rng.integers(0, 9, 20000),
         (rng.integers(1, 10 ** 8, 5000) + 0.5 + rng.choice([-1e-7, 1e-7, 3e-7, -3e-7], 5000)) / 10.0 ** rng.integers(0, 9, 5000)])
-    vals = np.concatenate([np.array(fixed), rnd]).astype("<f8")
+    return np.concatenate([np.array(fixed), rnd]).astype("<f8")
+
+
+def test_dtoa_g_p8_matches_reference_function(golden_dir, tmp_path):
+    """The 8-digit formatter behind --make-grm-sparse, byte for byte against the reference's own dtoa_g_p8
+    (2.0/include/plink2_string.cc:2641) on dtoa_p8_inputs(); tests/golden/dtoa_g_p8.json holds the digest of the
+    reference's text (make_host_format_set.py)."""
+    vals = dtoa_p8_inputs()
     vals.tofile(tmp_path / "in.bin")
-    subprocess.run([str(exe), str(tmp_path / "in.bin"), str(tmp_path / "ref.txt")], check=True)
     subprocess.run([BIN, "--debug-dtoa-p8", str(tmp_path / "in.bin"), str(tmp_path / "got.txt")], check=True)
-    ref = open(tmp_path / "ref.txt").read().split("\n")
-    got = open(tmp_path / "got.txt").read().split("\n")
-    assert len(ref) == len(got) == len(vals) + 1
-    assert ref == got
-    assert ref[10] == "123456.79" and ref[17] == "0.66666667" and ref[22] == " inf"
+    want = json.load(open(os.path.join(golden_dir, "dtoa_g_p8.json")))
+    raw = open(tmp_path / "got.txt", "rb").read()
+    got = raw.decode().split("\n")
+    assert want["lines"] == len(vals) and len(got) == len(vals) + 1
+    assert got[10] == "123456.79" and got[17] == "0.66666667" and got[22] == " inf"
+    assert hashlib.sha256(raw).hexdigest() == want["sha256"]
 
 
-@pytest.mark.skipif(not (os.path.isdir(REF_INC) and os.path.exists(SFMT_OBJ)), reason="needs the reference's compiled SFMT (this container only)")
-def test_sfmt_and_gaussian_fill_match_reference_generator(tmp_path):
+def test_sfmt_and_gaussian_fill_match_reference_generator(golden_dir, tmp_path):
     """The SFMT-19937 restatement and FillGaussian reproduce the reference's vendored generator
-    (2.0/include/SFMT.c) and RandNormal/FillGaussianDArr (2.0/plink2_random.cc:29-99) bit for bit."""
-    harness = tmp_path / "h.c"
-    harness.write_text(r'''
-#include <stdio.h>
-#include <stdlib.h>
-#include <math.h>
-#include "SFMT.h"
-int main(int argc, char** argv) {
-  sfmt_t s; uint32_t seed = strtoul(argv[1], 0, 10); unsigned long n = strtoul(argv[2], 0, 10);
-  sfmt_init_gen_rand(&s, seed);
-  FILE* f = fopen(argv[3], "wb");
-  for (unsigned long k = 0; k < n; ++k) { uint32_t v = sfmt_genrand_uint32(&s); fwrite(&v, 4, 1, f); }
-  fclose(f);
-  /* second stream: init_by_array with the next four draws, as InitAllocSfmtpArr does */
-  uint32_t key[4]; for (int k = 0; k < 4; ++k) key[k] = sfmt_genrand_uint32(&s);
-  sfmt_t t; sfmt_init_by_array(&t, key, 4);
-  f = fopen(argv[4], "wb");
-  for (unsigned long k = 0; k < 1000; ++k) { uint32_t v = sfmt_genrand_uint32(&t); fwrite(&v, 4, 1, f); }
-  fclose(f);
-  return 0;
-}
-''')
-    exe = tmp_path / "h"
-    subprocess.run(["gcc", "-O1", "-DSFMT_MEXP=19937", "-I" + REF_INC, str(harness), SFMT_OBJ, "-lm", "-o", str(exe)], check=True)
-    n = 5000
-    subprocess.run([str(exe), "11", str(n), str(tmp_path / "ref.u32"), str(tmp_path / "ref2.u32")], check=True)
+    (2.0/include/SFMT.c; its first draws for seed 11 are tests/golden/sfmt_seed11.u32, make_host_format_set.py) and
+    RandNormal/FillGaussianDArr (2.0/plink2_random.cc:29-99) bit for bit."""
+    n = SFMT_DRAWS
     subprocess.run([BIN, "--debug-sfmt", "11", str(n), str(tmp_path / "got.u32")], check=True)
-    ref = np.fromfile(tmp_path / "ref.u32", dtype=np.uint32)
+    ref = np.fromfile(os.path.join(golden_dir, "sfmt_seed11.u32"), dtype="<u4")
     got = np.fromfile(tmp_path / "got.u32", dtype=np.uint32)
-    assert np.array_equal(ref, got)
+    assert ref.size == n and np.array_equal(ref, got)
     # Gaussian fill, single stream: Box-Muller on consecutive draws
     subprocess.run([BIN, "--debug-gauss", "11", "1000", "1", str(tmp_path / "g.f64")], check=True)
     g = np.fromfile(tmp_path / "g.f64", dtype=np.float64)
@@ -452,8 +420,8 @@ def test_variant_id_templates(tmp_path):
 def test_make_pgen_writes_a_fileset_every_reader_accepts(tmp_path):
     """--make-pgen: fixed-width .pgen (storage mode 0x02) + .pvar + .psam of the filtered view.  The text files are the
     reference's byte for byte (column rules: FID / PAT+MAT / CM / PHENO1 only when informative); the .pgen is read
-    back by this program's own reader - and by the reference binary when it is available in the checkout - and must
-    reproduce the .bed the reference wrote for the same view."""
+    back by this program's own reader and must reproduce the .bed the reference wrote for the same view.  The .pgen itself is the one the reference writes for the
+    same view in the same storage mode (`--make-pgen format=2`), byte for byte."""
     gd = os.path.join(ROOT, "tests", "golden")
     out = str(tmp_path / "o")
     r = subprocess.run([BIN, "--bfile", "x", "--keep", "x_keep1.txt", "x_keep2.txt", "--extract", "x_extract.txt", "--make-pgen", "--out", out], capture_output=True, text=True, cwd=gd)
@@ -465,10 +433,7 @@ def test_make_pgen_writes_a_fileset_every_reader_accepts(tmp_path):
     back = str(tmp_path / "back")
     r = subprocess.run([BIN, "--pfile", out, "--make-bed", "--out", back], capture_output=True, text=True)
     assert r.returncode == 0 and open(back + ".bed", "rb").read() == open(os.path.join(gd, "x_mp.bed"), "rb").read()
-    ref = os.path.join(ROOT, "oracle", "_ref", "plink2")
-    if os.path.exists(ref):
-        r = subprocess.run([ref, "--pfile", out, "--make-bed", "--out", back + "_ref"], capture_output=True, text=True)
-        assert r.returncode == 0 and open(back + "_ref.bed", "rb").read() == open(os.path.join(gd, "x_mp.bed"), "rb").read()
+    assert raw == open(os.path.join(gd, "x_mp.pgen"), "rb").read()
     r = subprocess.run([BIN, "--pedmap", "p", "--make-pgen", "--out", out], capture_output=True, text=True, cwd=gd)
     assert r.returncode == 0, r.stdout + r.stderr
     for ext in ("pvar", "psam"):  # CM column (a nonzero centimorgan exists), PAT / MAT columns, NA sex and phenotype

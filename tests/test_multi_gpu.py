@@ -1,17 +1,18 @@
 """GPU (needs >= 2 devices; skipped on a 1-GPU box): the multi-GPU product path - `plink2_b200 --gpus 2` splits the
 N x N triangle into tile-aligned row slabs, every device uploads half of each decoded block and NCCL (inside
-libpl2gpu) all-gathers the column tile.  Outputs must be byte-identical to the single-GPU run and to the reference."""
+libpl2gpu) all-gathers the column tile.  Outputs must be byte-identical to the single-GPU run and to the reference
+(its results for the seeded input are kept in tests/golden, see test_scale_gpu.py)."""
 import os
 import subprocess
 
 import numpy as np
 import pytest
 
+from test_scale_gpu import _write_bed, assert_grm_matches_sample, dataset, gold, sha256
+
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "plink_ng_b200", "plink2_b200")
-REF = os.path.join(ROOT, "oracle", "_ref", "plink2")
-REF_LAPACK = os.path.join(ROOT, "oracle", "_ref", "plink2_lapack")
 
 
 def _device_count():
@@ -30,52 +31,29 @@ def sh(cmd):
 def dummy(tmp_path_factory):
     if _device_count() < 2:
         pytest.skip("needs two CUDA devices")
-    d = tmp_path_factory.mktemp("mg")
-    pre = str(d / "d")
-    sh([REF, "--dummy", "3000", "20000", "0.02", "--seed", "11", "--threads", "4", "--make-bed", "--out", pre])
-    return pre
+    return dataset(tmp_path_factory.mktemp("mg"), "mg")
 
 
 def test_king_two_gpus_byte_identical(dummy, tmp_path):
     flags = ["--make-king", "bin", "triangle", "--make-king-table", "counts", "--king-table-filter", "-0.03"]
-    ref, one, two = str(tmp_path / "ref"), str(tmp_path / "one"), str(tmp_path / "two")
-    sh([REF, "--bfile", dummy] + flags + ["--threads", "8", "--out", ref])
+    one, two = str(tmp_path / "one"), str(tmp_path / "two")
     sh([BIN, "--bfile", dummy] + flags + ["--out", one])
     r = sh([BIN, "--bfile", dummy] + flags + ["--gpus", "2", "--out", two])
     assert "reduced to 1" not in r.stdout
     for ext in (".king.bin", ".kin0", ".king.id"):
-        a = open(ref + ext, "rb").read()
-        assert a == open(one + ext, "rb").read(), ext
-        assert a == open(two + ext, "rb").read(), ext
+        want = gold("mg")["king"][ext[1:]]
+        assert sha256(one + ext) == want, ext
+        assert sha256(two + ext) == want, ext
 
 
 def test_grm_two_gpus_matches_single(dummy, tmp_path):
-    one, two, ref = str(tmp_path / "one"), str(tmp_path / "two"), str(tmp_path / "ref")
-    sh([REF_LAPACK, "--bfile", dummy, "--make-grm-bin", "--threads", "8", "--out", ref])
+    one, two = str(tmp_path / "one"), str(tmp_path / "two")
     sh([BIN, "--bfile", dummy, "--make-grm-bin", "--out", one])
     sh([BIN, "--bfile", dummy, "--make-grm-bin", "--gpus", "2", "--out", two])
     for ext in (".grm.bin", ".grm.N.bin", ".grm.id"):
         assert open(one + ext, "rb").read() == open(two + ext, "rb").read(), ext
-    a = np.fromfile(ref + ".grm.bin", dtype=np.float32).astype(np.float64)
-    b = np.fromfile(two + ".grm.bin", dtype=np.float32).astype(np.float64)
-    assert np.allclose(b, a, rtol=1e-5, atol=2e-8)
-    assert open(ref + ".grm.N.bin", "rb").read() == open(two + ".grm.N.bin", "rb").read()
-
-
-def _write_bed(prefix, geno):
-    """geno [variants, samples] codes 0/1/2/3 (ALT count, 3 = missing) -> .bed (SNP-major) / .bim / .fam."""
-    m, n = geno.shape
-    bed_code = np.array([3, 2, 0, 1], dtype=np.uint8)[geno]  # .bed: 00 hom A1(=ALT), 01 missing, 10 het, 11 hom A2(=REF)
-    pad = (-n) % 4
-    b = np.pad(bed_code, ((0, 0), (0, pad))).reshape(m, -1, 4)
-    packed = (b[:, :, 0] | (b[:, :, 1] << 2) | (b[:, :, 2] << 4) | (b[:, :, 3] << 6)).astype(np.uint8)
-    with open(prefix + ".bed", "wb") as f:
-        f.write(bytes([0x6C, 0x1B, 0x01]))
-        packed.tofile(f)
-    with open(prefix + ".bim", "w") as f:
-        f.write("".join(f"1\tsnp{k}\t0\t{k + 1}\tA\tG\n" for k in range(m)))
-    with open(prefix + ".fam", "w") as f:
-        f.write("".join(f"0\tper{k}\t0\t0\t2\t-9\n" for k in range(n)))
+    assert_grm_matches_sample(two + ".grm.bin", 3000, "scale_mg_grm_sample.npz")
+    assert sha256(two + ".grm.N.bin") == gold("mg")["grm.N.bin"]
 
 
 def test_pca_approx_two_gpus_matches_single(tmp_path):

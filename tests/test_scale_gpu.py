@@ -1,12 +1,16 @@
 """GPU: parity AT SCALE, through the product (the plink2_b200 host program), against the UNMODIFIED reference
-binary run on this box on the same files (oracle/_ref/plink2[_lapack], built by oracle/build_ref.sh; it
-travels to the GPU box with the snapshot).  Inputs come from the reference's own generator
-(`--dummy`, 2.0/plink2_import.cc:16326-16460) so both programs read identical bytes.
+binary.  The inputs are regenerated from a seed (the LD generator of test_ld_gpu.py, written as .bed); what the
+reference wrote for the same files is kept in tests/golden/scale_ref.json (SHA-256 digests of the files that must
+match byte for byte, row counts, the table filter) and tests/golden/scale_*_grm_sample.npz (a fixed sample of the
+GRM entries that are compared within a tolerance); tests/golden/make_scale_set.py regenerates both from
+oracle/_ref/plink2[_lapack].
 
 Sizes are the ones SURVEY.md 8(c) names for the smoke set: 4,096 samples x 65,536 variants (32 row tiles x
 up to 52 column tiles, two 32,768-variant batches for GRM / several for KING), plus a 20,000-sample KING
 run (157 row tiles) that pins tile placement and orientation pair by pair, and a forced multipass run.
 """
+import hashlib
+import json
 import os
 import re
 import subprocess
@@ -17,10 +21,55 @@ import pytest
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "plink_ng_b200", "plink2_b200")
-REF = os.path.join(ROOT, "oracle", "_ref", "plink2")
-REF_LAPACK = os.path.join(ROOT, "oracle", "_ref", "plink2_lapack")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 ENV = dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0])
-THREADS = str(max(1, min(32, len(os.sched_getaffinity(0)))))
+
+# name -> (samples, variants, seed)
+DATASETS = {"d4k": (4096, 65536, 1), "d20k": (20000, 2048, 5), "d3k": (3000, 4096, 9), "mg": (3000, 20000, 11)}
+
+
+def _write_bed(prefix, geno):
+    """geno [variants, samples] codes 0/1/2/3 (ALT count, 3 = missing) -> .bed (SNP-major) / .bim / .fam."""
+    m, n = geno.shape
+    bed_code = np.array([3, 2, 0, 1], dtype=np.uint8)[geno]  # .bed: 00 hom A1(=ALT), 01 missing, 10 het, 11 hom A2(=REF)
+    pad = (-n) % 4
+    b = np.pad(bed_code, ((0, 0), (0, pad))).reshape(m, -1, 4)
+    packed = (b[:, :, 0] | (b[:, :, 1] << 2) | (b[:, :, 2] << 4) | (b[:, :, 3] << 6)).astype(np.uint8)
+    with open(prefix + ".bed", "wb") as f:
+        f.write(bytes([0x6C, 0x1B, 0x01]))
+        packed.tofile(f)
+    with open(prefix + ".bim", "w") as f:
+        f.write("".join(f"1\tsnp{k}\t0\t{k + 1}\tA\tG\n" for k in range(m)))
+    with open(prefix + ".fam", "w") as f:
+        f.write("".join(f"0\tper{k}\t0\t0\t2\t-9\n" for k in range(n)))
+
+
+def write_dataset(name, prefix):
+    from test_ld_gpu import _ld_geno
+
+    n, m, seed = DATASETS[name]
+    _write_bed(prefix, _ld_geno(m, n, seed=seed))
+
+
+def sha256(path):
+    h = hashlib.sha256()
+    with open(path, "rb") as f:
+        for chunk in iter(lambda: f.read(1 << 24), b""):
+            h.update(chunk)
+    return h.hexdigest()
+
+
+def gold(name):
+    with open(os.path.join(GOLDEN, "scale_ref.json")) as f:
+        return json.load(f)[name]
+
+
+def dataset(tmp_dir, name):
+    """The seeded input fileset; its .bed must be the one the reference results were computed on."""
+    pre = str(tmp_dir / name)
+    write_dataset(name, pre)
+    assert sha256(pre + ".bed") == gold(name)["bed"], f"{name}: the generator no longer writes the input the reference results belong to"
+    return pre
 
 
 def sh(cmd, env=None, ok=(0,)):
@@ -29,84 +78,59 @@ def sh(cmd, env=None, ok=(0,)):
     return r
 
 
-def need(path):
-    if not os.path.exists(path):
-        pytest.fail(f"{path} is missing: run oracle/build_ref.sh where /root/reference exists (it travels with the snapshot)")
+def assert_same(got, digest, what):
+    assert sha256(got) == digest, f"{got} differs from the reference's {what}"
 
 
-def same_file(a, b, chunk=1 << 26):
-    if os.path.getsize(a) != os.path.getsize(b):
-        return False
-    with open(a, "rb") as fa, open(b, "rb") as fb:
-        while True:
-            x, y = fa.read(chunk), fb.read(chunk)
-            if x != y:
-                return False
-            if not x:
-                return True
-
-
-def assert_same_text(ref, got):
-    """Byte-identical text files; on mismatch say where (line counts, first differing line)."""
-    if same_file(ref, got):
-        return
-    a, b = open(ref, "rb").read().split(b"\n"), open(got, "rb").read().split(b"\n")
-    k = next((i for i, (x, y) in enumerate(zip(a, b)) if x != y), min(len(a), len(b)))
-    ndiff = sum(1 for x, y in zip(a, b) if x != y)
-    raise AssertionError(f"{got} differs from {ref}: {len(a)} vs {len(b)} lines, {ndiff} differing among the common ones, first at line {k + 1}:\n"
-                         f"  ref: {a[k][:200] if k < len(a) else None}\n  got: {b[k][:200] if k < len(b) else None}\n"
-                         f"  ref prev: {a[k - 1][:200] if k else None}\n  ref next: {a[k + 1][:200] if k + 1 < len(a) else None}\n  got next: {b[k + 1][:200] if k + 1 < len(b) else None}")
+def assert_grm_matches_sample(path, n, sample):
+    """fp32 .grm.bin entries at the stored positions within 1e-5 relative of the reference's (LAPACK build, fp64 dsyrk)."""
+    got = np.fromfile(path, dtype=np.float32)
+    assert got.size == n * (n + 1) // 2
+    with np.load(os.path.join(GOLDEN, sample)) as z:
+        idx, want = z["index"].astype(np.int64), z["value"].astype(np.float64)
+    # fp32 payload: half an ulp of the stored value (6e-8 relative) on top of the 1e-5 relative contract
+    b = got[idx].astype(np.float64)
+    assert np.allclose(b, want, rtol=1e-5, atol=2e-8), float(np.max(np.abs(want - b)))
 
 
 @pytest.fixture(scope="module")
 def dummy4k(tmp_path_factory):
-    need(REF)
-    d = tmp_path_factory.mktemp("scale4k")
-    pre = str(d / "d")
-    sh([REF, "--dummy", "4096", "65536", "0.01", "--seed", "1", "--threads", "4", "--make-bed", "--out", pre])
-    return pre
+    return dataset(tmp_path_factory.mktemp("scale4k"), "d4k")
 
 
 def test_king_table_and_matrix_4096x65536_byte_identical(dummy4k, tmp_path):
     """Every .kin0 count column (NSNP HETHET IBS0 HET1_HOM2 HET2_HOM1 IBS KINSHIP) on a NON-EMPTY filtered table
-    (>= 1e5 rows) plus the whole fp32 kinship triangle, byte for byte."""
-    ref, out = str(tmp_path / "ref"), str(tmp_path / "b200")
-    sh([REF, "--bfile", dummy4k, "--make-king", "bin4", "triangle", "--threads", THREADS, "--out", ref])
-    kin = np.fromfile(ref + ".king.bin", dtype=np.float32)
-    assert kin.size == 4096 * 4095 // 2
-    thr = repr(float(np.quantile(kin.astype(np.float64), 0.97)))
-    flags = ["--make-king-table", "counts", "cols=+ibs1,+ibs", "--king-table-filter", thr]
-    sh([REF, "--bfile", dummy4k] + flags + ["--threads", THREADS, "--out", ref])
+    (>= 1e5 rows, the top 3 % of the reference's kinship values) plus the whole fp32 kinship triangle, byte for byte."""
+    want = gold("d4k")["king_table"]
+    out = str(tmp_path / "b200")
+    flags = ["--make-king-table", "counts", "cols=+ibs1,+ibs", "--king-table-filter", want["king_table_filter"]]
     sh([BIN, "--bfile", dummy4k] + flags + ["--make-king", "bin4", "triangle", "--out", out], env=ENV)
-    rows = sum(1 for _ in open(ref + ".kin0")) - 1
-    assert rows >= 100_000, rows
-    assert same_file(ref + ".king.bin", out + ".king.bin")
-    assert same_file(ref + ".king.id", out + ".king.id")
-    assert_same_text(ref + ".kin0", out + ".kin0")
+    rows = sum(1 for _ in open(out + ".kin0")) - 1
+    assert rows == want["kin0_rows"] >= 100_000, rows
+    assert os.path.getsize(out + ".king.bin") == 4 * (4096 * 4095 // 2)
+    assert_same(out + ".king.bin", want["king.bin"], ".king.bin")
+    assert_same(out + ".king.id", want["king.id"], ".king.id")
+    assert_same(out + ".kin0", want["kin0"], ".kin0")
 
 
 def test_king_matrix_20000_samples_pairwise(tmp_path):
     """157 row tiles x up to 250 column tiles: the whole 2e8-pair fp32 kinship triangle against the reference's, so a
     tile-placement or orientation error anywhere in the triangle fails (the marginal-sum test cannot see those)."""
-    need(REF)
-    pre, ref, out = str(tmp_path / "d"), str(tmp_path / "ref"), str(tmp_path / "b200")
-    sh([REF, "--dummy", "20000", "2048", "0.02", "--seed", "5", "--threads", "4", "--make-bed", "--out", pre])
-    sh([REF, "--bfile", pre, "--make-king", "bin4", "triangle", "--threads", THREADS, "--out", ref])
+    pre, out = dataset(tmp_path, "d20k"), str(tmp_path / "b200")
     sh([BIN, "--bfile", pre, "--make-king", "bin4", "triangle", "--out", out], env=ENV)
-    assert os.path.getsize(ref + ".king.bin") == 4 * (20000 * 19999 // 2)
-    assert same_file(ref + ".king.bin", out + ".king.bin")
+    assert os.path.getsize(out + ".king.bin") == 4 * (20000 * 19999 // 2)
+    assert_same(out + ".king.bin", gold("d20k")["king.bin"], ".king.bin")
 
 
 def test_king_forced_multipass_matches_single_pass(tmp_path):
     """--gpu-memory caps the device budget so RunKing needs >= 3 row-block passes (the reference's
     CountTrianglePasses behaviour, 2.0/plink2_matrix_calc.cc:216-255); outputs must not change."""
-    need(REF)
-    pre, ref, one = str(tmp_path / "d"), str(tmp_path / "ref"), str(tmp_path / "one")
-    sh([REF, "--dummy", "3000", "4096", "0.02", "--seed", "9", "--threads", "4", "--make-bed", "--out", pre])
+    pre, one = dataset(tmp_path, "d3k"), str(tmp_path / "one")
+    want = gold("d3k")
     flags = ["--make-king", "bin", "triangle", "--make-king-table", "counts", "--king-table-filter", "-0.05"]
-    sh([REF, "--bfile", pre] + flags + ["--threads", THREADS, "--out", ref])
     sh([BIN, "--bfile", pre] + flags + ["--out", one], env=ENV)
-    assert same_file(ref + ".king.bin", one + ".king.bin") and same_file(ref + ".kin0", one + ".kin0")
+    assert_same(one + ".king.bin", want["king.bin"], ".king.bin")
+    assert_same(one + ".kin0", want["kin0"], ".kin0")
     passes = 0
     for mib in (640, 560, 500, 470, 450, 435, 425, 415):
         multi = str(tmp_path / f"multi{mib}")
@@ -115,36 +139,32 @@ def test_king_forced_multipass_matches_single_pass(tmp_path):
             break  # below the fixed staging buffers: nothing smaller can work
         m = re.search(r"(\d+) passes over the variants", r.stdout)
         passes = int(m.group(1)) if m else 1
-        assert same_file(ref + ".king.bin", multi + ".king.bin"), mib
-        assert same_file(ref + ".kin0", multi + ".kin0"), mib
+        assert_same(multi + ".king.bin", want["king.bin"], f".king.bin (--gpu-memory {mib})")
+        assert_same(multi + ".kin0", want["kin0"], f".kin0 (--gpu-memory {mib})")
         if passes >= 3:
             break
     assert passes >= 3, f"no --gpu-memory value produced >= 3 passes (last: {passes})"
 
 
 def test_grm_4096x65536_vs_reference_blas(dummy4k, tmp_path):
-    """.grm.bin against the LAPACK build of the reference (threaded OpenBLAS dsyrk in fp64) within 1e-5 relative,
-    .grm.N.bin (per-pair observation counts) and .grm.id exactly."""
-    need(REF_LAPACK)
-    ref, out = str(tmp_path / "ref"), str(tmp_path / "b200")
-    sh([REF_LAPACK, "--bfile", dummy4k, "--make-grm-bin", "--threads", THREADS, "--out", ref])
+    """.grm.bin against the LAPACK build of the reference (threaded OpenBLAS dsyrk in fp64) within 1e-5 relative on
+    every diagonal entry and 4,096 fixed off-diagonal ones (a misplaced 128 x 128 tile is hit with probability
+    0.9997), .grm.N.bin (per-pair observation counts) and .grm.id
+    exactly."""
+    want = gold("d4k")["grm"]
+    out = str(tmp_path / "b200")
     sh([BIN, "--bfile", dummy4k, "--make-grm-bin", "--out", out], env=ENV)
-    a = np.fromfile(ref + ".grm.bin", dtype=np.float32).astype(np.float64)
-    b = np.fromfile(out + ".grm.bin", dtype=np.float32).astype(np.float64)
-    assert a.size == b.size == 4096 * 4097 // 2
-    # fp32 payload: half an ulp of the stored value (6e-8 relative) on top of the 1e-5 relative contract
-    assert np.allclose(b, a, rtol=1e-5, atol=2e-8), float(np.max(np.abs(a - b)))
-    assert same_file(ref + ".grm.N.bin", out + ".grm.N.bin")
-    assert same_file(ref + ".grm.id", out + ".grm.id")
+    assert_grm_matches_sample(out + ".grm.bin", 4096, "scale_d4k_grm_sample.npz")
+    assert_same(out + ".grm.N.bin", want["grm.N.bin"], ".grm.N.bin")
+    assert_same(out + ".grm.id", want["grm.id"], ".grm.id")
 
 
 def test_indep_pairwise_500_50_02_keep_list_4096x65536(dummy4k, tmp_path):
     """The BASELINE config-4 command on the 65,536-variant set: .prune.in / .prune.out byte-identical."""
-    ref, out = str(tmp_path / "ref"), str(tmp_path / "b200")
-    flags = ["--indep-pairwise", "500", "50", "0.2"]
-    sh([REF, "--bfile", dummy4k] + flags + ["--threads", THREADS, "--out", ref])
-    sh([BIN, "--bfile", dummy4k] + flags + ["--out", out], env=ENV)
-    kept = sum(1 for _ in open(ref + ".prune.in"))
-    assert 10_000 < kept < 60_000, kept
-    assert same_file(ref + ".prune.in", out + ".prune.in")
-    assert same_file(ref + ".prune.out", out + ".prune.out")
+    want = gold("d4k")["prune"]
+    out = str(tmp_path / "b200")
+    sh([BIN, "--bfile", dummy4k, "--indep-pairwise", "500", "50", "0.2", "--out", out], env=ENV)
+    kept = sum(1 for _ in open(out + ".prune.in"))
+    assert 10_000 < want["kept"] < 60_000 and kept == want["kept"], kept
+    assert_same(out + ".prune.in", want["prune.in"], ".prune.in")
+    assert_same(out + ".prune.out", want["prune.out"], ".prune.out")
