@@ -265,8 +265,14 @@ int pl2gpu_score_end(Pl2ScoreJob* job);
  * This is the roofline denominator bench.py reports against. ---- */
 int pl2gpu_int8_peak(Pl2GpuCtx* ctx, uint32_t n_cols, int form, double min_seconds, double* tops_out, double* seconds_out);
 
-/* ---- self-test of the tcgen05 operand path (descriptor/layout probe); returns 0 iff an int8
- * UMMA over library-written shared-memory tiles reproduces a scalar device-side reference. ---- */
+/* ---- measured block-scaled FP4 tensor peak: as pl2gpu_int8_peak's form 1, with tcgen05.mma kind::mxf4
+ * (E2M1 operands, UE8M0 scales, M = 128, N = n_cols, K = 64, A operand in tensor memory as king_ts_kernel uses it);
+ * *tops_out = 2*128*n_cols*64 ops x UMMAs / elapsed, in TOP/s. ---- */
+int pl2gpu_mxf4_peak(Pl2GpuCtx* ctx, uint32_t n_cols, double min_seconds, double* tops_out, double* seconds_out);
+
+/* ---- self-test of the tcgen05 operand path (descriptor/layout probe); returns 0 iff int8 UMMAs (both
+ * operands in shared memory, and A in tensor memory) and kind::mxf4 UMMAs in king_ts_kernel's operand layout
+ * reproduce a scalar reference, and the kind::mxf4 F32 accumulator adds +-1 exactly past 2^20. ---- */
 int pl2gpu_selftest_umma(Pl2GpuCtx* ctx, int verbose);
 /* Debug probe used by tests to pin the operand layout: runs `k_steps` int8 UMMAs (M = 128) over the
  * given shared-memory images / descriptor fields and returns D as int32 [128][n] (host memory). */

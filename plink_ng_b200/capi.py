@@ -82,6 +82,7 @@ SIGNATURES = {
     "pl2gpu_score_end": (C.c_int, [vp]),
     "pl2_ld_prune_walk": (C.c_int, [C.c_uint32, vp, vp, C.c_uint32, C.c_uint32, C.c_int, vp, vp, vp, C.c_uint32, C.c_uint32, vp]),
     "pl2gpu_int8_peak": (C.c_int, [vp, C.c_uint32, C.c_int, C.c_double, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+    "pl2gpu_mxf4_peak": (C.c_int, [vp, C.c_uint32, C.c_double, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "pl2gpu_selftest_umma": (C.c_int, [vp, C.c_int]),
     "pl2gpu_debug_umma": (
         C.c_int,

@@ -51,6 +51,26 @@ constexpr uint32_t kTabMiss = 0x01000000u;    // mu: missing indicator
 // vector register for the whole kernel.
 __device__ __forceinline__ uint32_t table_reg(uint32_t table, uint32_t thread_zero) { return table | thread_zero; }
 
+// ---- 2-bit genotype -> E2M1 nibble planes (kind::mxf4 operands) ----
+// Every plane value is 0, +1 or -1, exact in E2M1 (1.0 = 0x2, -1.0 = 0xA).  One 32-bit word of 16 codes becomes two
+// words of 8 nibbles: word 0 holds the even samples (codes 0, 2, .., 14), word 1 the odd ones.  That K permutation is
+// harmless as long as BOTH operands of a product go through this function: the dot product is order-free.
+struct Nib3 {
+  uint32_t het[2], hom[2], sgn[2];  // planes T, H, S with the meaning of kTabHet / kTabHom / kTabSgn
+};
+__device__ __forceinline__ Nib3 expand_nibbles(uint32_t w) {
+  Nib3 r;
+  const uint32_t x[2] = {w & 0x33333333u, (w >> 2) & 0x33333333u};  // code c in bits [0,2) of each nibble
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const uint32_t b0 = x[h] & 0x11111111u, b1 = (x[h] >> 1) & 0x11111111u;
+    r.het[h] = (b0 & ~b1) << 1;                          // code 1
+    r.hom[h] = (b0 ^ 0x11111111u) << 1;                  // codes 0 and 2
+    r.sgn[h] = r.hom[h] | (((b0 ^ 0x11111111u) & b1) << 3);  // code 0 -> +1 (0x2), code 2 -> -1 (0xA)
+  }
+  return r;
+}
+
 // MN-major, no-swizzle UMMA operand tile ("interleave" canonical layout,
 // cute/atom/mma_traits_sm100.hpp:171): 16 consecutive samples of one variant are one 16-byte row
 // of an 8-row core matrix (8 consecutive variants, 128 contiguous bytes); core matrices step by

@@ -16,10 +16,10 @@ constexpr uint32_t kTsKcJ = 64;         // variants per shared-memory stage (two
 constexpr uint32_t kTsRawBoxBytes = 32; // inner extent of the TMA box over the raw block (>= 20 bytes = 80 samples, multiple of 16)
 
 // ---- operand re-tiling of the staged block raw[variant][pitch] (2-bit, variant-major) -------------
-// Both copies make every producer load of king_ts_kernel a contiguous run of bytes (the first TS
-// version read 8 bytes per lane from 32 different rows: 336 L1 wavefronts per k-step, LSU-bound).
+// Sample-major copies make every producer load of the TS kernels a contiguous run of bytes (the first
+// TS version read 8 bytes per lane from 32 different rows: 336 L1 wavefronts per k-step, LSU-bound).
 //
-// Row side:  raw_i[row tile rt][k-step ks][row 0..127][8 bytes]   8 bytes = 32 variants of one sample
+// GRM / PCA row side (int8 k-steps of 32 variants):  raw_i[row tile rt][k-step ks][row 0..127][8 bytes]   8 bytes = 32 variants of one sample
 // One CTA = 64 variants x 64 samples through a shared-memory byte tile.
 // Only samples [s_base, s_base + 64 * gridDim.y) are written (a job re-tiles its own row tiles only);
 // row tile s_base / 128 is stored at index 0.
@@ -41,6 +41,29 @@ static __global__ void __launch_bounds__(256) geno_tile_rows_kernel(const uint8_
     for (uint32_t j = 0; j < 16; ++j) w |= static_cast<uint32_t>(tile[16 * vw + j][sl]) << (2 * j);
     const uint32_t s = s0 + sl, v = v0 + 16 * vw;
     *reinterpret_cast<uint32_t*>(raw_i + (static_cast<uint64_t>((s - s_base) >> 7) * kstep_ct + (v >> 5)) * 1024 + (s & 127) * 8 + 4 * ((v >> 4) & 1)) = w;
+  }
+}
+
+// Sample-major copy for 64-variant k-steps (king_ts_kernel.cuh):  raw_x[k-step ks][sample s][16 bytes]
+// 16 bytes = 64 variants of one sample, variant 64 ks + j at bits [2 (j % 16), 2 (j % 16) + 2) of word j / 16.
+// Samples [0, gridDim.y * 64) are written; one CTA = 64 variants x 64 samples through a shared-memory byte tile.
+static __global__ void __launch_bounds__(256) geno_tile_samples_kernel(const uint8_t* __restrict__ raw, uint32_t pitch, uint32_t sample_ct_x, uint8_t* __restrict__ raw_x) {
+  __shared__ uint8_t tile[64][68];
+  const uint32_t v0 = blockIdx.x * 64, s0 = blockIdx.y * 64;
+  const uint32_t t = threadIdx.x;
+  {
+    const uint32_t v = t >> 2, sw = t & 3;
+    const uint32_t w = *reinterpret_cast<const uint32_t*>(raw + static_cast<uint64_t>(v0 + v) * pitch + s0 / 4 + 4 * sw);
+#pragma unroll
+    for (uint32_t j = 0; j < 16; ++j) tile[v][16 * sw + j] = static_cast<uint8_t>((w >> (2 * j)) & 3u);
+  }
+  __syncthreads();
+  {
+    const uint32_t sl = t >> 2, vw = t & 3;
+    uint32_t w = 0;
+#pragma unroll
+    for (uint32_t j = 0; j < 16; ++j) w |= static_cast<uint32_t>(tile[16 * vw + j][sl]) << (2 * j);
+    *reinterpret_cast<uint32_t*>(raw_x + (static_cast<uint64_t>(blockIdx.x) * sample_ct_x + s0 + sl) * 16 + 4 * vw) = w;
   }
 }
 

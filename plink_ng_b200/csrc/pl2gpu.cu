@@ -102,19 +102,42 @@ void FreeTileList(TileList* tl) {
 }
 
 // ---- TMA tensor maps ----
-int MakeRawTensorMap(CUtensorMap* out, void* base, uint32_t pitch, uint32_t rows, uint32_t box_bytes, uint32_t box_rows) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn encode = nullptr;
+typedef CUresult (*TensorMapEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+static TensorMapEncodeFn GetTensorMapEncode() {
+  static TensorMapEncodeFn encode = nullptr;
   if (!encode) {
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn) {
       cudaGetLastError();
       set_error("cuTensorMapEncodeTiled is not available from this driver");
-      return 1;
+      return nullptr;
     }
-    encode = reinterpret_cast<EncodeFn>(fn);
+    encode = reinterpret_cast<TensorMapEncodeFn>(fn);
   }
+  return encode;
+}
+
+// 3-D uint8 tensor map over a sample-major copy raw_x[kstep_ct][sample_ct][16] (geno_tile_samples_kernel) with box
+// {16, box_samples, box_ksteps}: one TMA copy lands box_ksteps consecutive [box_samples][16] blocks in shared memory.
+static int MakeSampleMajorTensorMap(CUtensorMap* out, void* base, uint32_t sample_ct, uint32_t kstep_ct, uint32_t box_samples, uint32_t box_ksteps) {
+  const TensorMapEncodeFn encode = GetTensorMapEncode();
+  if (!encode) return 1;
+  const cuuint64_t dims[3] = {16, sample_ct, kstep_ct};
+  const cuuint64_t strides[2] = {16, 16ull * sample_ct};  // bytes, dimensions 1 and 2
+  const cuuint32_t box[3] = {16, box_samples, box_ksteps};
+  const cuuint32_t elem_strides[3] = {1, 1, 1};
+  const CUresult r = encode(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, base, dims, strides, box, elem_strides, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled failed (%d) for a %u-sample x %u-k-step copy", static_cast<int>(r), sample_ct, kstep_ct);
+    return 1;
+  }
+  return 0;
+}
+
+int MakeRawTensorMap(CUtensorMap* out, void* base, uint32_t pitch, uint32_t rows, uint32_t box_bytes, uint32_t box_rows) {
+  const TensorMapEncodeFn encode = GetTensorMapEncode();
+  if (!encode) return 1;
   const cuuint64_t dims[2] = {pitch, rows};
   const cuuint64_t strides[1] = {pitch};  // bytes, dimension 1
   const cuuint32_t box[2] = {box_bytes, box_rows};
@@ -246,12 +269,13 @@ struct Pl2KingJob {
   uint32_t sample_ct = 0, row_start = 0, row_end = 0;
   int algo = kPl2KingAlgoTensor;
   TileList tiles;
-  // TS path: two staged blocks + two row-side re-tiled copies, so that the copy / all-gather, padding and
-  // row re-tiling of batch k+1 (prep stream) overlap the tensor kernel of batch k (compute stream).
+  // TS path: two staged blocks + two sample-major copies, so that the copy / all-gather, padding and
+  // re-tiling of batch k+1 (prep stream) overlap the tensor kernel of batch k (compute stream).
   // The other algorithms use buffer 0 on the compute stream only.
   GenoStage stage[2];
-  uint8_t* d_raw_t[2] = {nullptr, nullptr};  // TS path: row-side re-tiled copy of the job's own row tiles (geno_tile.cuh)
-  CUtensorMap tmap[2];                       // TS path: 2-D tensor maps over stage[b].d_raw for the column-side TMA loads
+  uint8_t* d_raw_t[2] = {nullptr, nullptr};  // TS path: sample-major copy of samples [0, ts_samples) (geno_tile_samples_kernel)
+  uint32_t ts_samples = 0;                   // TS path: samples in that copy, a multiple of kTsSamplePad covering the row tiles
+  CUtensorMap tmap_i[2], tmap_j[2];          // TS path: 3-D tensor maps over d_raw_t[b], row-tile and column-tile boxes
   cudaEvent_t ev_prep_done[2] = {nullptr, nullptr};
   cudaEvent_t ev_kernel_start[2] = {nullptr, nullptr};  // timing-enabled pair around the tensor kernel (pl2gpu_king_last_kernel_ms)
   cudaEvent_t ev_kernel_done[2] = {nullptr, nullptr};
@@ -460,11 +484,12 @@ uint64_t pl2gpu_king_mem_required(uint32_t sample_ct, uint32_t row_start, uint32
   const uint64_t tiles = CountTiles(row_start, row_end, false);
   const uint64_t npad = RoundUpU32(sample_ct, kSamplePad);
   const uint64_t need_ss = tiles * kKingTileAccWords * 4 + cap * (npad / 4) + 3ull * (cap / 32) * npad * 4 + tiles * 16;
-  // TS tensor (the default): 128 x 64 tiles, two raw blocks + two row-side re-tiled copies of the job's row tiles
+  // TS tensor (the default): 128 x 80 tiles, two raw blocks + two sample-major copies of samples [0, row_end)
+  // (a row block's column tiles reach back to sample 0)
   const uint64_t tiles_ts = CountTiles(row_start, row_end, false, kTsCols);
   const uint64_t npad_ts = RoundUpU32(sample_ct, kTsSamplePad);
-  const uint64_t row_tiles = row_end > row_start ? (DivUpU32(row_end, kTileRows) - row_start / kTileRows) : 0;
-  const uint64_t need_ts = tiles_ts * kTsTileAccWords * 4 + 2 * cap * (npad_ts / 4) + 2 * row_tiles * kTileRows * (cap / 4) + tiles_ts * 16;
+  const uint64_t copy_samples = row_end > row_start ? RoundUpU32(row_end, kTsSamplePad) : 0;
+  const uint64_t need_ts = tiles_ts * kTsTileAccWords * 4 + 2 * cap * (npad_ts / 4) + 2 * copy_samples * (cap / 4) + tiles_ts * 16;
   return (need_ss > need_ts ? need_ss : need_ts) + kKingOutStageBytes + slack;
 }
 
@@ -512,14 +537,18 @@ int pl2gpu_king_begin_ex(Pl2GpuCtx* ctx, uint32_t sample_ct, uint32_t row_start,
   if (BuildTileList(row_start, row_end, false, &job->tiles, job->tile_cols)) return fail();
   for (int b = 0; b < (ts ? 2 : 1); ++b) {
     if (StageAlloc(sample_ct, cap, &job->stage[b], ts ? kTsSamplePad : kSamplePad)) return fail();
-    if (ts) {
-      const uint64_t raw_t_bytes = static_cast<uint64_t>(job->tiles.row_tile_ct) * kTileRows * (job->stage[b].variant_cap / 4);
-      if (cudaMalloc(&job->d_raw_t[b], raw_t_bytes ? raw_t_bytes : 16) != cudaSuccess) {
+    if (ts && job->tiles.tile_ct) {
+      // the row tiles end at or before sample_ct_padded (a multiple of kTsSamplePad), so the copy fits the stage
+      job->ts_samples = RoundUpU32((job->tiles.row_tile_first + job->tiles.row_tile_ct) * kTileRows, kTsSamplePad);
+      const uint32_t ksteps = job->stage[b].variant_cap / kTsKstep;
+      if (cudaMalloc(&job->d_raw_t[b], static_cast<uint64_t>(job->ts_samples) * (job->stage[b].variant_cap / 4)) != cudaSuccess) {
         cudaGetLastError();
-        set_error("pl2gpu_king_begin: insufficient device memory for the row-side re-tiled genotype copy");
+        set_error("pl2gpu_king_begin: insufficient device memory for the sample-major genotype copy");
         return fail();
       }
-      if (MakeRawTensorMap(&job->tmap[b], job->stage[b].d_raw, job->stage[b].pitch, job->stage[b].variant_cap, kTsRawBoxBytes, 2 * kTsKcJ)) return fail();
+      if (MakeSampleMajorTensorMap(&job->tmap_i[b], job->d_raw_t[b], job->ts_samples, ksteps, kTileRows, kTsRingKsteps) ||
+          MakeSampleMajorTensorMap(&job->tmap_j[b], job->d_raw_t[b], job->ts_samples, ksteps, kTsCols, kTsRingKsteps))
+        return fail();
     }
   }
   const uint64_t acc_bytes = static_cast<uint64_t>(job->tiles.tile_ct) * (5ull * job->tile_cols * kTileRows) * sizeof(int32_t);
@@ -550,8 +579,8 @@ int pl2gpu_king_begin_ex(Pl2GpuCtx* ctx, uint32_t sample_ct, uint32_t row_start,
   return 0;
 }
 
-// TS path: the staged block stage[b] holds `cur` variants (rows [0, cur)); pad it, re-tile the job's row
-// tiles and queue the tensor kernel.  Everything up to the kernel runs on the prep stream.
+// TS path: the staged block stage[b] holds `cur` variants (rows [0, cur)); pad it, re-tile samples
+// [0, ts_samples) sample-major and queue the tensor kernel.  Everything up to the kernel runs on the prep stream.
 static int KingTsPrepAndLaunch(Pl2KingJob* job, uint32_t b, uint32_t cur, bool pad_valid_rows) {
   Ctx* c = &job->ctx->c;
   cudaStream_t prep = c->copy_stream;
@@ -568,13 +597,13 @@ static int KingTsPrepAndLaunch(Pl2KingJob* job, uint32_t b, uint32_t cur, bool p
     job->kernel_pending[b] = true;
     return 0;
   }
-  geno_tile_rows_kernel<<<dim3(padded / 64, job->tiles.row_tile_ct * (kTileRows / 64)), 256, 0, prep>>>(st.d_raw, st.pitch, padded / 32, job->tiles.row_tile_first * kTileRows, job->d_raw_t[b]);
+  geno_tile_samples_kernel<<<dim3(padded / kTsKstep, job->ts_samples / 64), 256, 0, prep>>>(st.d_raw, st.pitch, job->ts_samples, job->d_raw_t[b]);
   c->launches++;
   PL2_CUDA_OK(cudaGetLastError());
   PL2_CUDA_OK(cudaEventRecord(job->ev_prep_done[b], prep));
   PL2_CUDA_OK(cudaStreamWaitEvent(c->stream, job->ev_prep_done[b], 0));
   PL2_CUDA_OK(cudaEventRecord(job->ev_kernel_start[b], c->stream));
-  king_ts_kernel<<<job->tiles.tile_ct, kTsThreads, kTsSmemBytes, c->stream>>>(job->tmap[b], job->d_raw_t[b], job->tiles.row_tile_first, padded, job->tiles.d_tile_order, job->tiles.d_tile_rt, job->tiles.d_tile_tc, job->d_raw_acc);
+  king_ts_kernel<<<job->tiles.tile_ct, kTsThreads, kTsSmemBytes, c->stream>>>(job->tmap_i[b], job->tmap_j[b], padded, job->tiles.d_tile_order, job->tiles.d_tile_rt, job->tiles.d_tile_tc, job->d_raw_acc);
   c->launches++;
   PL2_CUDA_OK(cudaGetLastError());
   PL2_CUDA_OK(cudaEventRecord(job->ev_kernel_done[b], c->stream));
@@ -1060,6 +1089,139 @@ int pl2gpu_debug_umma(Pl2GpuCtx* ctx, const uint8_t* a_img, uint32_t a_bytes, co
   return 0;
 }
 
+// kind::mxf4 checks behind king_ts_kernel (umma_probe.cuh):
+//  * layout: random 0/+-1 operands, M = 128, N = 160, two k-steps of K = 64; A rows in tensor memory with element k
+//    in nibble k % 2 (low first) of byte k / 2, B K-major in king_ts_kernel's core-matrix arrangement (K chunk of
+//    32 at kTsLboJ-style stride, 8-sample groups at kCoreBytes), unit scales at tensor-memory columns [496, 512);
+//  * precision: the F32 accumulator must add single +-1 products exactly once it has passed 2^20, the largest count
+//    one launch can reach.
+static int SelftestMxf4(Pl2GpuCtx* ctx, int verbose) {
+  Ctx* c = &ctx->c;
+  PL2_CUDA_OK(cudaFuncSetAttribute(umma_probe_mxf4_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kProbeSmemBytes));
+  PL2_CUDA_OK(cudaFuncSetAttribute(umma_mxf4_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kProbeSmemBytes));
+  constexpr uint32_t M = 128, N = 160, KS = 2, K = 64 * KS;
+  constexpr uint32_t lbo = (N / 8) * kCoreBytes + 64, step = 2 * lbo;
+  std::vector<int> av(M * K), bv(N * K);
+  uint32_t seed = 4242;
+  auto rnd = [&]() {
+    seed = seed * 1664525u + 1013904223u;
+    return static_cast<int>((seed >> 24) % 3) - 1;
+  };
+  auto nib = [](int v) -> uint32_t { return v == 0 ? 0u : (v > 0 ? 0x2u : 0xAu); };
+  for (auto& x : av) x = rnd();
+  for (auto& x : bv) x = rnd();
+  std::vector<uint8_t> a_rows(M * K / 2, 0), b(KS * step, 0);
+  for (uint32_t m = 0; m < M; ++m)
+    for (uint32_t k = 0; k < K; ++k) a_rows[m * (K / 2) + k / 2] |= nib(av[m * K + k]) << (4 * (k & 1));
+  for (uint32_t n = 0; n < N; ++n)
+    for (uint32_t k = 0; k < K; ++k) {
+      const uint32_t off = (k / 64) * step + ((k % 64) / 32) * lbo + (n / 8) * kCoreBytes + (n % 8) * 16 + (k % 32) / 2;
+      b[off] |= nib(bv[n * K + k]) << (4 * (k & 1));
+    }
+  UmmaProbeParams prm{};
+  prm.b_bytes = static_cast<uint32_t>(b.size());
+  prm.b_lbo = lbo;
+  prm.b_sbo = kCoreBytes;
+  prm.b_step_bytes = step;
+  prm.k_steps = KS;
+  prm.idesc = make_idesc_mxf4(M, N);
+  prm.n = N;
+  uint8_t *d_a = nullptr, *d_b = nullptr;
+  uint32_t* d_d = nullptr;
+  std::vector<uint32_t> d(M * N);
+  PL2_CUDA_OK(cudaMalloc(&d_a, a_rows.size()));
+  PL2_CUDA_OK(cudaMalloc(&d_b, b.size()));
+  PL2_CUDA_OK(cudaMalloc(&d_d, d.size() * 4));
+  PL2_CUDA_OK(cudaMemcpyAsync(d_a, a_rows.data(), a_rows.size(), cudaMemcpyHostToDevice, c->stream));
+  PL2_CUDA_OK(cudaMemcpyAsync(d_b, b.data(), b.size(), cudaMemcpyHostToDevice, c->stream));
+  umma_probe_mxf4_ts_kernel<<<1, 128, kProbeSmemBytes, c->stream>>>(d_a, d_b, prm, d_d);
+  c->launches++;
+  PL2_CUDA_OK(cudaGetLastError());
+  PL2_CUDA_OK(cudaMemcpyAsync(d.data(), d_d, d.size() * 4, cudaMemcpyDeviceToHost, c->stream));
+  PL2_CUDA_OK(cudaStreamSynchronize(c->stream));
+  uint32_t bad = 0;
+  for (uint32_t m = 0; m < M; ++m)
+    for (uint32_t n = 0; n < N; ++n) {
+      int ref = 0;
+      for (uint32_t k = 0; k < K; ++k) ref += av[m * K + k] * bv[n * K + k];
+      float got;
+      memcpy(&got, &d[m * N + n], 4);
+      if (got != static_cast<float>(ref)) {
+        if (verbose && bad < 8) fprintf(stderr, "selftest_umma(mxf4) mismatch m=%u n=%u got=%g want=%d\n", m, n, got, ref);
+        ++bad;
+      }
+    }
+  // precision: 2^20 / 64 + 1 all-ones UMMAs, then five single +-1 products (umma_mxf4_exact_kernel)
+  uint32_t bad_exact = 0;
+  const uint32_t base = (1u << 20) / 64 + 1;
+  umma_mxf4_exact_kernel<<<1, 128, kProbeSmemBytes, c->stream>>>(base, lbo, kCoreBytes, d_d);
+  c->launches++;
+  PL2_CUDA_OK(cudaGetLastError());
+  PL2_CUDA_OK(cudaMemcpyAsync(d.data(), d_d, 128 * 16 * 4, cudaMemcpyDeviceToHost, c->stream));
+  PL2_CUDA_OK(cudaStreamSynchronize(c->stream));
+  for (uint32_t m = 0; m < 128; ++m)
+    for (uint32_t n = 0; n < 16; ++n) {
+      int64_t want = 64ll * base + 1;
+      for (uint32_t j = 1; j <= 4; ++j) want += ((n >> (j - 1)) & 1) ? -1 : 1;
+      float got;
+      memcpy(&got, &d[m * 16 + n], 4);
+      if (static_cast<double>(got) != static_cast<double>(want)) {
+        if (verbose && bad_exact < 8) fprintf(stderr, "selftest_umma(mxf4 precision) m=%u n=%u got=%.1f want=%lld\n", m, n, got, static_cast<long long>(want));
+        ++bad_exact;
+      }
+    }
+  cudaFree(d_a);
+  cudaFree(d_b);
+  cudaFree(d_d);
+  if (bad) {
+    set_error("pl2gpu_selftest_umma: kind::mxf4 TS form: %u of %u accumulator entries differ from the scalar reference", bad, M * N);
+    return 1;
+  }
+  if (bad_exact) {
+    set_error("pl2gpu_selftest_umma: kind::mxf4 accumulator is not exact past 2^20 (%u of 2048 entries differ)", bad_exact);
+    return 1;
+  }
+  return 0;
+}
+
+int pl2gpu_mxf4_peak(Pl2GpuCtx* ctx, uint32_t n_cols, double min_seconds, double* tops_out, double* seconds_out) {
+  if (!ctx || !tops_out || n_cols < 16 || n_cols > 240 || (n_cols & 15)) {
+    set_error("pl2gpu_mxf4_peak: bad arguments (n_cols must be a multiple of 16 in [16,240])");
+    return 1;
+  }
+  Ctx* c = &ctx->c;
+  PL2_CUDA_OK(cudaSetDevice(c->device));
+  PL2_CUDA_OK(cudaFuncSetAttribute(umma_mxf4_peak_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kProbeSmemBytes));
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  PL2_CUDA_OK(cudaEventCreate(&e0));
+  PL2_CUDA_OK(cudaEventCreate(&e1));
+  const uint32_t blocks = 4096;  // x 32 UMMAs x 2 issuer warps
+  const double ops_per_launch = 2.0 * 128 * n_cols * 64 * 32.0 * 2 * blocks * c->sm_count;
+  umma_mxf4_peak_kernel<<<c->sm_count, 128, kProbeSmemBytes, c->stream>>>(n_cols, blocks);  // warm-up
+  c->launches++;
+  PL2_CUDA_OK(cudaStreamSynchronize(c->stream));
+  double total_s = 0, total_ops = 0;
+  const uint32_t per_batch = 8;
+  while (total_s < min_seconds) {
+    PL2_CUDA_OK(cudaEventRecord(e0, c->stream));
+    for (uint32_t k = 0; k < per_batch; ++k) umma_mxf4_peak_kernel<<<c->sm_count, 128, kProbeSmemBytes, c->stream>>>(n_cols, blocks);
+    c->launches += per_batch;
+    PL2_CUDA_OK(cudaEventRecord(e1, c->stream));
+    PL2_CUDA_OK(cudaEventSynchronize(e1));
+    PL2_CUDA_OK(cudaGetLastError());
+    float ms = 0;
+    PL2_CUDA_OK(cudaEventElapsedTime(&ms, e0, e1));
+    total_s += ms * 1e-3;
+    total_ops += ops_per_launch * per_batch;
+    if (min_seconds <= 0) break;
+  }
+  cudaEventDestroy(e0);
+  cudaEventDestroy(e1);
+  *tops_out = total_ops / total_s / 1e12;
+  if (seconds_out) *seconds_out = total_s;
+  return 0;
+}
+
 int pl2gpu_selftest_umma(Pl2GpuCtx* ctx, int verbose) {
   if (getenv("PL2_UMMA_BENCH")) {  // diagnostic: tcgen05.mma issue / execution rate (umma_probe.cuh)
     Ctx* c = &ctx->c;
@@ -1163,6 +1325,7 @@ int pl2gpu_selftest_umma(Pl2GpuCtx* ctx, int verbose) {
       return 3;
     }
   }
+  PL2_TRY(SelftestMxf4(ctx, verbose));
   return 0;
 }
 

@@ -59,6 +59,9 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
 __device__ __forceinline__ void tma_load_2d(uint32_t dst_smem, const void* tensor_map, int32_t c0, int32_t c1, uint64_t* bar) {
   asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst_smem), "l"(tensor_map), "r"(c0), "r"(c1), "r"(smem_u32(bar)) : "memory");
 }
+__device__ __forceinline__ void tma_load_3d(uint32_t dst_smem, const void* tensor_map, int32_t c0, int32_t c1, int32_t c2, uint64_t* bar) {
+  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(dst_smem), "l"(tensor_map), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar)) : "memory");
+}
 // 1-D bulk copy global -> shared (SASS UBLKCP); bytes and both addresses multiples of 16.
 __device__ __forceinline__ void bulk_load_1d(uint32_t dst_smem, const void* src, uint32_t bytes, uint64_t* bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_smem), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
@@ -94,6 +97,18 @@ __device__ __forceinline__ uint2 lds64(uint32_t addr) {
   uint2 v;
   asm volatile("ld.shared.v2.b32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(addr) : "memory");
   return v;
+}
+__device__ __forceinline__ uint4 lds128(uint32_t addr) {
+  uint4 v;
+  asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr) : "memory");
+  return v;
+}
+__device__ __forceinline__ void sts64x2(uint32_t addr, uint32_t lo, uint32_t hi) { asm volatile("st.shared.v2.b32 [%0], {%1,%2};" ::"r"(addr), "r"(lo), "r"(hi) : "memory"); }
+// F32 accumulator bits -> int32, round to nearest (exact for the integer values below 2^24 the FP4 kernels produce)
+__device__ __forceinline__ int32_t f32_bits_to_s32_rn(uint32_t bits) {
+  int32_t r;
+  asm("cvt.rni.s32.f32 %0, %1;" : "=r"(r) : "f"(__uint_as_float(bits)));
+  return r;
 }
 
 // ---------------- fences ----------------
@@ -189,6 +204,30 @@ __device__ __forceinline__ void umma_i8_ts(uint32_t d_tmem, uint32_t a_tmem, uin
       : "r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+
+// Instruction descriptor for kind::mxf4 (block-scaled E2M1, PTX ISA tcgen05 "instruction descriptor" table for
+// the .kind::mxf8f6f4 / .kind::mxf4 forms):
+//   [4,6) SF id of B (byte of the scale column)   [7,10) A format: 1 = E2M1   [10,12) B format: 1 = E2M1
+//   [15] / [16] A / B major: 0 = K-major (the only layout 4-bit operands accept)
+//   [17,23) N >> 3   [23] scale format: 1 = UE8M0   [24,29) M >> 4   [29,31) SF id of A   [31] K = 64
+// D is always F32.  Callers that fill every scale byte with the same value can leave both SF ids at 0.
+__host__ __device__ constexpr uint32_t make_idesc_mxf4(uint32_t m, uint32_t n) {
+  return (1u << 7) | (1u << 10) | ((n >> 3) << 17) | (1u << 23) | ((m >> 4) << 24);
+}
+
+// D[tmem] (+)= (A[tmem] x 2^sfa) * (B[smem] x 2^sfb), K = 64 packed E2M1 per row (32 bytes = 8 TMEM columns of A),
+// one UE8M0 scale per 32 K (scale_vec::2X) read from tensor memory at sfa / sfb; issued by ONE thread.
+__device__ __forceinline__ void umma_mxf4_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t sfa_tmem, uint32_t sfb_tmem, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %6, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.scale_vec::2X [%0], [%1], %2, %3, [%4], [%5], p;\n\t}"
+      :
+      : "r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(sfa_tmem), "r"(sfb_tmem), "r"(accumulate)
+      : "memory");
+}
+// UE8M0 scale bytes of 2^0 (bias 127): with every scale byte set to this, a block-scaled product is the plain product
+constexpr uint32_t kUe8m0One4 = 0x7F7F7F7Fu;
 
 // registers -> TMEM: thread t of the warp writes 8 consecutive 32-bit columns of lane (lane base + t)
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {

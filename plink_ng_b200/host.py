@@ -88,6 +88,12 @@ class GpuContext:
         check(lib.pl2gpu_int8_peak(self._h, n_cols, form, min_seconds, C.byref(tops), C.byref(secs)), "pl2gpu_int8_peak")
         return float(tops.value), float(secs.value)
 
+    def mxf4_peak(self, n_cols: int = 160, min_seconds: float = 2.0):
+        """Measured chip-wide tcgen05 kind::mxf4 rate (TOP/s, seconds), A operand in tensor memory."""
+        tops, secs = C.c_double(), C.c_double()
+        check(lib.pl2gpu_mxf4_peak(self._h, n_cols, min_seconds, C.byref(tops), C.byref(secs)), "pl2gpu_mxf4_peak")
+        return float(tops.value), float(secs.value)
+
     def comm_init(self, rank: int, world: int, unique_id: bytes):
         """Attach an NCCL communicator (collective over all ranks; rank 0 makes the id with comm_unique_id())."""
         buf = (C.c_uint8 * 128).from_buffer_copy(unique_id)
