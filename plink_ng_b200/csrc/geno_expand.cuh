@@ -52,22 +52,39 @@ constexpr uint32_t kTabMiss = 0x01000000u;    // mu: missing indicator
 __device__ __forceinline__ uint32_t table_reg(uint32_t table, uint32_t thread_zero) { return table | thread_zero; }
 
 // ---- 2-bit genotype -> E2M1 nibble planes (kind::mxf4 operands) ----
-// Every plane value is 0, +1 or -1, exact in E2M1 (1.0 = 0x2, -1.0 = 0xA).  One 32-bit word of 16 codes becomes two
-// words of 8 nibbles: word 0 holds the even samples (codes 0, 2, .., 14), word 1 the odd ones.  That K permutation is
-// harmless as long as BOTH operands of a product go through this function: the dot product is order-free.
+// Every plane value is 0, +1 or -1, exact in E2M1 (1.0 = 0x2, -1.0 = 0xA, and 0x8 = -0.0).  The kind::mxf4 kernels
+// read a sample-major copy (geno_tile_samples_kernel) whose bits are laid out so that the per-tile decode is a few
+// masks: every tile decodes every word again, about a thousand times more often than the copy is written.
+//
+// A word of the copy holds 16 variants v + 0..15 of one sample.  Each variant is a pair (p, q) with
+//   p = 1 for hom-REF and hom-ALT (the H plane; the magnitude of the S plane),
+//   q = 1 for het and hom-ALT (the sign bit of the S plane),
+// so code 0 -> (1, 0), 1 -> (0, 1), 2 -> (1, 1), 3 (missing, padding) -> (0, 0): an all-zero copy is all missing.
+// Nibble i holds variant v + i in bits 1 (p) and 3 (q), and variant v + 8 + i in bits 0 (p) and 2 (q).  Then
+//   S = W & 0xAAAAAAAA   (hom-REF 0x2 = +1, hom-ALT 0xA = -1, het 0x8 = -0, missing 0)
+//   H = W & 0x22222222,  T = ~W & (W >> 2) & 0x22222222   (het = q and not p)
+// for variants v + 0..7, and the same on W << 1 for variants v + 8..15: 9 instructions per 16 variants.
+__host__ __device__ constexpr uint32_t mxf4_copy_bits(uint32_t code, uint32_t j) {  // variant j (0..15) of a word
+  const uint32_t p = ~code & 1u, q = (code ^ (code >> 1)) & 1u;
+  const uint32_t sh = 4 * (j & 7) + (j < 8 ? 1 : 0);
+  return (p << sh) | (q << (sh + 2));
+}
+// One word of the copy -> two words of 8 E2M1 nibbles per plane: word 0 = variants v + 0..7, word 1 = v + 8..15,
+// nibble i = variant v + i or v + 8 + i (low nibble first), i.e. K order = variant order.  Both operands of every
+// product go through this function.
 struct Nib3 {
-  uint32_t het[2], hom[2], sgn[2];  // planes T, H, S with the meaning of kTabHet / kTabHom / kTabSgn
+  uint32_t het[2], hom[2], sgn[2];  // planes T, H, S with the values of kTabHet / kTabHom / kTabSgn
 };
-__device__ __forceinline__ Nib3 expand_nibbles(uint32_t w) {
+__host__ __device__ __forceinline__ Nib3 decode_mxf4(uint32_t w) {
+  constexpr uint32_t kMag = 0x22222222u, kMagSign = 0xAAAAAAAAu;
   Nib3 r;
-  const uint32_t x[2] = {w & 0x33333333u, (w >> 2) & 0x33333333u};  // code c in bits [0,2) of each nibble
-#pragma unroll
-  for (int h = 0; h < 2; ++h) {
-    const uint32_t b0 = x[h] & 0x11111111u, b1 = (x[h] >> 1) & 0x11111111u;
-    r.het[h] = (b0 & ~b1) << 1;                          // code 1
-    r.hom[h] = (b0 ^ 0x11111111u) << 1;                  // codes 0 and 2
-    r.sgn[h] = r.hom[h] | (((b0 ^ 0x11111111u) & b1) << 3);  // code 0 -> +1 (0x2), code 2 -> -1 (0xA)
-  }
+  const uint32_t w1 = w << 1;
+  r.sgn[0] = w & kMagSign;
+  r.hom[0] = w & kMag;
+  r.het[0] = ~w & (w >> 2) & kMag;
+  r.sgn[1] = w1 & kMagSign;
+  r.hom[1] = w1 & kMag;
+  r.het[1] = ~w1 & (w >> 1) & kMag;
   return r;
 }
 

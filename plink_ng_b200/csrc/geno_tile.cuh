@@ -3,6 +3,7 @@
 // shared memory.  Kernels are static (header is included by several translation units).
 #pragma once
 #include "common.cuh"
+#include "geno_expand.cuh"
 
 namespace pl2 {
 
@@ -45,7 +46,8 @@ static __global__ void __launch_bounds__(256) geno_tile_rows_kernel(const uint8_
 }
 
 // Sample-major copy for 64-variant k-steps (king_ts_kernel.cuh):  raw_x[k-step ks][sample s][16 bytes]
-// 16 bytes = 64 variants of one sample, variant 64 ks + j at bits [2 (j % 16), 2 (j % 16) + 2) of word j / 16.
+// 16 bytes = 64 variants of one sample; word j / 16 holds variant 64 ks + j in the decode-friendly bit order of
+// geno_expand.cuh (mxf4_copy_bits: variant j % 16 < 8 in bits 1 and 3 of nibble j % 8, else in bits 0 and 2).
 // Samples [0, gridDim.y * 64) are written; one CTA = 64 variants x 64 samples through a shared-memory byte tile.
 static __global__ void __launch_bounds__(256) geno_tile_samples_kernel(const uint8_t* __restrict__ raw, uint32_t pitch, uint32_t sample_ct_x, uint8_t* __restrict__ raw_x) {
   __shared__ uint8_t tile[64][68];
@@ -62,7 +64,7 @@ static __global__ void __launch_bounds__(256) geno_tile_samples_kernel(const uin
     const uint32_t sl = t >> 2, vw = t & 3;
     uint32_t w = 0;
 #pragma unroll
-    for (uint32_t j = 0; j < 16; ++j) w |= static_cast<uint32_t>(tile[16 * vw + j][sl]) << (2 * j);
+    for (uint32_t j = 0; j < 16; ++j) w |= mxf4_copy_bits(tile[16 * vw + j][sl], j);
     *reinterpret_cast<uint32_t*>(raw_x + (static_cast<uint64_t>(blockIdx.x) * sample_ct_x + s0 + sl) * 16 + 4 * vw) = w;
   }
 }

@@ -39,8 +39,12 @@ constexpr uint32_t kTsSfCol = kTsAccCols + kTsASlots * kTsASlotCols;  // 496
 static_assert(kTsSfCol + 16 <= 512, "TMEM budget: accumulators + A slots + scale columns");
 // B stage (one k-step), K-major no-swizzle: a core matrix is 8 samples x 16 bytes (32 K).  K chunk kc (0, 1) holds
 // the 30 eight-sample groups [T 0..9 | H 0..9 | S 0..9] at kCoreBytes apart; the +64 makes the two chunks' rows
-// fall in different bank halves, so the column warps' 8-byte stores are conflict-free.
+// fall in different bank halves, so the column warps' 8-byte stores are conflict-free.  The column warps and the
+// issuer hand the stages over two k-steps at a time (one wait, fence and arrive per two k-steps); deeper stages
+// would not leave room for two CTAs per SM.
 constexpr uint32_t kTsStagesJ = 4;
+constexpr uint32_t kTsHandJ = 2;                  // k-steps per B-stage handshake
+constexpr uint32_t kTsBarsJ = kTsStagesJ / kTsHandJ;
 constexpr uint32_t kTsLboJ = 3 * (kTsCols / 8) * kCoreBytes + 64;  // 3904: K-chunk stride
 constexpr uint32_t kTsStageBytesJ = 2 * kTsLboJ;                    // 7808
 constexpr uint32_t kTsRingKsteps = 4;                              // k-steps per TMA copy (one ring slot)
@@ -63,8 +67,8 @@ king_ts_kernel(const __grid_constant__ CUtensorMap tmap_i, const __grid_constant
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ __align__(8) uint64_t bar_full_a[kTsASlots];
   __shared__ __align__(8) uint64_t bar_empty_a[kTsASlots];
-  __shared__ __align__(8) uint64_t bar_full_b[kTsStagesJ];
-  __shared__ __align__(8) uint64_t bar_empty_b[kTsStagesJ];
+  __shared__ __align__(8) uint64_t bar_full_b[kTsBarsJ];
+  __shared__ __align__(8) uint64_t bar_empty_b[kTsBarsJ];
   __shared__ __align__(8) uint64_t bar_full_rj[kTsRawJSlots];
   __shared__ __align__(8) uint64_t bar_empty_rj[kTsRawJSlots];
   __shared__ __align__(8) uint64_t bar_full_ri[kTsRawISlots];
@@ -87,7 +91,7 @@ king_ts_kernel(const __grid_constant__ CUtensorMap tmap_i, const __grid_constant
       mbar_init(&bar_full_a[s], 4);             // one arrival per row-side warp of the owning group
       mbar_init(&bar_empty_a[s], 1);
     }
-    for (uint32_t s = 0; s < kTsStagesJ; ++s) {
+    for (uint32_t s = 0; s < kTsBarsJ; ++s) {
       mbar_init(&bar_full_b[s], kTsColWarps);
       mbar_init(&bar_empty_b[s], 1);
     }
@@ -139,7 +143,7 @@ king_ts_kernel(const __grid_constant__ CUtensorMap tmap_i, const __grid_constant
       const uint32_t words[4] = {w.x, w.y, w.z, w.w};
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
-        const Nib3 n = expand_nibbles(words[i]);
+        const Nib3 n = decode_mxf4(words[i]);
         e.v[0][2 * i] = n.het[0]; e.v[0][2 * i + 1] = n.het[1];
         e.v[1][2 * i] = n.hom[0]; e.v[1][2 * i + 1] = n.hom[1];
         e.v[2][2 * i] = n.sgn[0]; e.v[2][2 * i + 1] = n.sgn[1];
@@ -161,12 +165,12 @@ king_ts_kernel(const __grid_constant__ CUtensorMap tmap_i, const __grid_constant
     };
     Words words = load_slot(0);
     ExpI cur = expand_i(words.w[0]);
+    static_assert(kTsASlots == kTsRingKsteps, "k-step 4 q + grp + 2 h always uses A slot grp + 2 h");
     for (uint32_t q = 0; q < slot_iters; ++q) {
 #pragma unroll
       for (uint32_t h = 0; h < 2; ++h) {
-        const uint32_t ks = 4 * q + grp + 2 * h;
-        const uint32_t slot = ks % kTsASlots;
-        mbar_wait(&bar_empty_a[slot], ((ks / kTsASlots) & 1) ^ 1);
+        const uint32_t slot = grp + 2 * h;  // used for the q-th time
+        mbar_wait(&bar_empty_a[slot], (q & 1) ^ 1);
         tc_fence_after_sync();
         const uint32_t ta = taddr_lane + kTsAccCols + slot * kTsASlotCols;
         tmem_st8(ta, cur.v[0]);
@@ -205,18 +209,20 @@ king_ts_kernel(const __grid_constant__ CUtensorMap tmap_i, const __grid_constant
       uint32_t words[kTsRingKsteps];
 #pragma unroll
       for (uint32_t kk = 0; kk < kTsRingKsteps; ++kk) words[kk] = lds32(ring_j + sj * kTsRawJBytes + kk * (kTsCols * 16));
+      static_assert(kTsRingKsteps == kTsStagesJ, "one ring slot fills the B stages once");
 #pragma unroll
-      for (uint32_t kk = 0; kk < kTsRingKsteps; ++kk) {
-        const uint32_t it = kTsRingKsteps * q + kk;
-        const uint32_t sb = it % kTsStagesJ;
-        const Nib3 e = expand_nibbles(words[kk]);
-        mbar_wait(&bar_empty_b[sb], ((it / kTsStagesJ) & 1) ^ 1);
+      for (uint32_t sb = 0; sb < kTsStagesJ; ++sb) {
+        const uint32_t hb = sb / kTsHandJ;
+        const Nib3 e = decode_mxf4(words[sb]);
+        if (sb % kTsHandJ == 0) mbar_wait(&bar_empty_b[hb], (q & 1) ^ 1);
         const uint32_t a0 = smem_base + sb * kTsStageBytesJ + dst;
         sts64x2(a0, e.het[0], e.het[1]);
         sts64x2(a0 + kPlaneOff, e.hom[0], e.hom[1]);
         sts64x2(a0 + 2 * kPlaneOff, e.sgn[0], e.sgn[1]);
-        fence_proxy_async_smem();
-        mbar_arrive_warp(&bar_full_b[sb], lane);
+        if (sb % kTsHandJ == kTsHandJ - 1) {
+          fence_proxy_async_smem();
+          mbar_arrive_warp(&bar_full_b[hb], lane);
+        }
       }
       mbar_arrive_warp(&bar_empty_rj[sj], lane);  // every word went into an st.shared above
     }
@@ -234,7 +240,7 @@ king_ts_kernel(const __grid_constant__ CUtensorMap tmap_i, const __grid_constant
       const uint32_t ph = (it0 / kTsStagesJ) & 1;
 #pragma unroll
       for (uint32_t sb = 0; sb < kTsStagesJ; ++sb) {
-        mbar_wait(&bar_full_b[sb], ph);
+        if (sb % kTsHandJ == 0) mbar_wait(&bar_full_b[sb / kTsHandJ], ph);
         mbar_wait(&bar_full_a[sb], ph);
         tc_fence_after_sync();
         if (elect_one_sync()) {
@@ -246,7 +252,7 @@ king_ts_kernel(const __grid_constant__ CUtensorMap tmap_i, const __grid_constant
           umma_mxf4_ts(tmem_u + 2 * kTsCols, ta + 8, b_th, idesc_n160, sf, sf, acc);
           umma_mxf4_ts(tmem_u + 4 * kTsCols, ta + 16, b_s, idesc_n80, sf, sf, acc);
           umma_commit(&bar_empty_a[sb]);
-          umma_commit(&bar_empty_b[sb]);
+          if (sb % kTsHandJ == kTsHandJ - 1) umma_commit(&bar_empty_b[sb / kTsHandJ]);
         }
         __syncwarp();
       }
